@@ -238,8 +238,9 @@ class Harness:
         return float(ms.item()), kms, launches
 
 
-def measure_c1(hx, batch_per_gpu, K, W, want_kernel=True, want_e2e=True, want_sync=True):
-    """The C1 update on this rank's shard: returns dict(value-side timings, kernel ms, e2e timings, launches)."""
+def measure_c1(hx, batch_per_gpu, K, W, want_kernel=True, want_e2e=True, want_sync=True, dump_dir=None):
+    """The C1 update on this rank's shard: returns dict(value-side timings, kernel ms, e2e timings, launches).
+    With `dump_dir`, rank 0 writes the outputs of its last step there (dump_outputs)."""
     import torch
     from gops_b200.create_pkg.create_alg import create_alg
     from gops_b200 import _lib
@@ -276,7 +277,24 @@ def measure_c1(hx, batch_per_gpu, K, W, want_kernel=True, want_e2e=True, want_sy
     _lib.check(_lib.lib().gops_b200_plan_launch_info(plan.handle, info))
     out["launch"] = {"grid": info[0], "block": info[1], "tile_samples": info[2], "smem_bytes": info[3],
                      "kernel_path": alg.last_kernel_path()}
+    if dump_dir and hx.rank == 0:
+        dump_outputs(alg, dump_dir)
     return out
+
+
+def dump_outputs(alg, out_dir):
+    """What the last timed `local_update` left its caller, as float32 .npy files: the loss it computed (`loss.npy`;
+    with loss_lag = 1 the returned tb_info still carries the step before), every policy gradient
+    (`grad.<param>.npy`) and every updated policy parameter (`param.<param>.npy`).  All of it is a few KiB."""
+    import numpy as np
+    from gops_b200.utils.flat_params import GRAD_TAIL
+    os.makedirs(out_dir, exist_ok=True)
+    pol = alg.networks.policy
+    tail = pol.flat_params.gbuf[-GRAD_TAIL:].detach().cpu().numpy()
+    np.save(os.path.join(out_dir, "loss.npy"), tail[:1].astype(np.float32))
+    for name, p in pol.named_parameters():
+        np.save(os.path.join(out_dir, f"param.{name}.npy"), p.detach().cpu().numpy().astype(np.float32))
+        np.save(os.path.join(out_dir, f"grad.{name}.npy"), p.grad.detach().cpu().numpy().astype(np.float32))
 
 
 PATH_TEXT = {"tc": "tcgen05: BF16x3 UMMA for every dense product, weight gradients accumulate in TMEM",
@@ -411,6 +429,9 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-configs", action="store_true")
     ap.add_argument("--no-eager", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the loss, policy gradient and updated policy parameters of the "
+                         "last step as DIR/<name>.npy (inputs and initial weights are seeded: same arguments, same inputs)")
     args = ap.parse_args()
 
     rank = int(os.environ.get("RANK", "0"))
@@ -435,7 +456,7 @@ def main():
     Bglobal = args.global_batch
     per_gpu_strong = Bglobal // world
     main_b = per_gpu_strong if args.scaling == "strong" else Bglobal
-    m = measure_c1(hx, main_b, K, W)
+    m = measure_c1(hx, main_b, K, W, dump_dir=args.dump_outputs)
     other = None
     if world > 1:      # the other scaling mode, same run (value side only)
         other_b = Bglobal if args.scaling == "strong" else per_gpu_strong

@@ -4,10 +4,8 @@ can run on the GPU box, where /root/reference does not exist.
 TEST / MEASUREMENT INFRASTRUCTURE.  `oracle/_ref/` is git-ignored (no reference source enters the history) but not
 gpurun-ignored, so it travels with the snapshot like the built `.so`.  It is used by
   * `bench.py --impl reference`  (cpu_baseline.kind = "reference": the reference's own `alg.local_update` on the host
-    cores) and the `gpu_eager_baseline` leg (the same code with `use_gpu=True`, the "existing Blackwell path");
-  * `tests/test_gpu_reference_integration.py` (INTEGRATION.md's binding executed inside the real reference);
-  * `tests/test_oracle_vs_reference.py` (oracle restatement vs. the live reference on fresh inputs).
-Nothing under `gops_b200/` imports it.
+    cores) and the `gpu_eager_baseline` leg (the same code with `use_gpu=True`, the "existing Blackwell path").
+No test needs it, and nothing under `gops_b200/` imports it.
 
 Run:  python oracle/build_ref.py          (also called by __graft_entry__.build() when /root/reference exists)
 Copies  <reference>/gops/**/*.py  (+ the shipped FHADP idpendulum checkpoint and its config used as a known answer)

@@ -11,9 +11,8 @@ reference's own CPU path.  Gradients come from torch autograd exactly as in the 
 
 Parity pin: `oracle/make_golden.py` runs the UNMODIFIED reference (through `oracle/ref_shim.py`)
 in the build container and stores inputs / losses / gradients / post-Adam weights under
-`tests/golden/`; `tests/test_oracle_vs_golden.py` checks this file against those vectors, and
-`tests/test_oracle_vs_reference.py` checks it against the live reference when `/root/reference`
-is present.  Reference file:line citations are given per function (paths relative to the GOPS tree).
+`tests/golden/`; `tests/test_oracle_vs_golden.py` and `tests/test_oracle_vs_reference.py` check
+this file against those vectors.  Reference file:line citations are given per function (paths relative to the GOPS tree).
 """
 from __future__ import annotations
 

@@ -254,11 +254,65 @@ def run_detour():
     run_case("surrcstr_fhadpexterior", kw, d, [0, 1])
 
 
+def run_fresh_fhadp(H, B, seed):
+    """The reference's FHADP idpendulum update from its own initial weights on oracle-sampled inputs (a ninth of the
+    batch arriving done): initial policy, inputs, loss and gradients (tests/test_oracle_vs_reference.py)."""
+    from oracle import ref_runner
+    torch.set_num_threads(4)
+    torch.manual_seed(seed)
+    alg = ref_runner.create_reference_alg(ref_runner.c1_kwargs(H))
+    data = orc.sample_inputs("pyth_idpendulum", B, seed=seed)
+    data["done"][::9] = 1.0
+    rec = flat_inputs("pyth_idpendulum", data)
+    for k, v in _sd(alg).items():
+        rec["init/" + k] = v
+    tb = alg.local_update({k: v.clone() for k, v in data.items()}, 0)
+    rec["loss"] = np.float64(tb["Loss/Actor loss-RL iter"])
+    for pn, p in alg.networks.policy.named_parameters():
+        rec["grad/policy." + pn] = _np(p.grad).copy()
+    name = f"fresh_fhadp_idp_h{H}_b{B}_s{seed}"
+    np.savez_compressed(os.path.join(OUT, name + ".npz"), **rec)
+    print(name, float(rec["loss"]))
+
+
+def run_trainer_steps(n_steps=3, H=30, minibatch=512):
+    """Three OffSerialTrainer steps of the reference FHADP fed by the reference's own ReplayBuffer: initial state_dict,
+    the sampled minibatches, the loss of every step, and the policy's actions on 32 buffered observations after the
+    last step (tests/test_gpu_reference_integration.py)."""
+    from gops.trainer.buffer.replay_buffer import ReplayBuffer
+    from oracle import ref_runner
+    torch.manual_seed(11)
+    alg = ref_runner.create_reference_alg(ref_runner.c1_kwargs(H))
+    rec = {"init/" + k: v for k, v in _sd(alg).items()}
+    buf = ReplayBuffer(trainer="off_serial_trainer", seed=0, obsv_dim=6, action_dim=1, buffer_max_size=4096,
+                       additional_info={})
+    g = torch.Generator().manual_seed(3)
+    h = torch.tensor([5, 0.1, 0.1, 0.3, 0.3, 0.3])
+    obs = ((torch.rand(2048, 6, generator=g) * 2 - 1) * h).numpy()
+    buf.add_batch([(o, np.zeros(1, np.float32), 0.0, False, {}, o, {}, 0.0) for o in obs])
+    for it in range(n_steps):
+        replay = buf.sample_batch(minibatch)
+        for k, v in replay.items():
+            rec[f"it{it}/batch/{k}"] = _np(v).copy()
+        tb = alg.local_update({k: v.clone() for k, v in replay.items()}, it)
+        rec[f"it{it}/loss"] = np.float64(tb["Loss/Actor loss-RL iter"])
+    rec["act_obs"] = obs[:32].copy()
+    with torch.no_grad():
+        rec["act"] = _np(alg.networks.policy(torch.from_numpy(obs[:32]), 1)).copy()
+    np.savez_compressed(os.path.join(OUT, "trainer_steps_fhadp_idp_h30.npz"), **rec)
+    print("trainer_steps_fhadp_idp_h30", [float(rec[f"it{i}/loss"]) for i in range(n_steps)])
+
+
 def main():
     ref_shim.install()
     torch.set_num_threads(4)
     if "--detour" in sys.argv:
         run_detour()
+        return
+    if "--integration" in sys.argv:
+        run_fresh_fhadp(30, 64, 101)
+        run_fresh_fhadp(7, 33, 102)
+        run_trainer_steps()
         return
     run_dsac("dsac_idp")
     run_constrained()

@@ -1,9 +1,8 @@
 """Import shim that lets the UNMODIFIED reference (/root/reference, GOPS) be imported in this
 container, where gym / ray / matplotlib / ... are not installed.
 
-TEST INFRASTRUCTURE ONLY.  Used by `oracle/make_golden.py` (fixture generation) and by the
-`-m "not gpu"` tests that pin `oracle/gops_oracle.py` against the live reference when
-`/root/reference` exists.  Nothing in `gops_b200/` may import this file.
+TEST INFRASTRUCTURE ONLY.  Used by `oracle/make_golden.py` (fixture generation) and by
+`oracle/ref_runner.py` (bench.py's reference baselines).  Nothing in `gops_b200/` may import this file.
 
 Technique (SURVEY.md §8(c)): a `sys.meta_path` finder serves permissive stub modules for the
 missing third-party packages.  Lower-case attribute -> stub sub-module, Capitalised attribute ->

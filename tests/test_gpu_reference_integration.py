@@ -1,57 +1,50 @@
-"""INTEGRATION.md's binding executed INSIDE the real reference: `gops.create_pkg.create_alg.register` swaps the fused
-B200 algorithm into the reference's registry, the reference's own factory builds it, the reference's own ReplayBuffer
-(gops/trainer/buffer/replay_buffer.py) feeds it, and three OffSerialTrainer-style steps (off_serial_trainer.py:79-105:
-sample_batch -> .cuda() -> alg.local_update) run next to the unmodified reference algorithm on the same batches.
-Needs the reference tree (oracle/_ref on the GPU box, oracle/build_ref.py)."""
+"""INTEGRATION.md's binding: `create_alg.register` puts the fused B200 algorithm into a GOPS-style registry, the factory
+builds it from the reference's C1 keyword arguments, and three OffSerialTrainer-style steps (off_serial_trainer.py:79-105:
+sample_batch -> .cuda() -> alg.local_update) replay what the unmodified reference did on the same minibatches
+(tests/golden/trainer_steps_fhadp_idp_h30.npz, oracle/make_golden.py run_trainer_steps): the reference's initial
+state_dict, the minibatches its own ReplayBuffer sampled, its loss at every step and its policy's actions afterwards."""
 import numpy as np
 import pytest
 import torch
 
-from oracle import ref_runner, ref_shim
+from golden_util import load
+from oracle import ref_runner
 
-pytestmark = [pytest.mark.gpu, pytest.mark.skipif(not ref_shim.available(), reason="reference tree not reachable")]
+pytestmark = pytest.mark.gpu
 
 
 def test_register_binding_and_three_trainer_steps():
-    ref_shim.install()
-    from gops.create_pkg import create_alg as ref_ca
-    from gops.trainer.buffer.replay_buffer import ReplayBuffer
     from gops_b200.algorithm import fhadp as b200_fhadp
+    from gops_b200.create_pkg import create_alg as ca
 
-    H = 30
-    kw = ref_runner.c1_kwargs(H)
-    torch.manual_seed(11)
-    ref_alg = ref_ca.create_alg(**kw)                                  # the unmodified reference FHADP (CPU)
-    saved = ref_ca.registry["FHADP"]
+    rec = load("trainer_steps_fhadp_idp_h30")
+    ref_sd = {k[len("init/"):]: torch.from_numpy(v) for k, v in rec.items() if k.startswith("init/")}
+    kw = ref_runner.c1_kwargs(30)
+    saved = ca.registry["FHADP"]
     try:
-        ref_ca.register("FHADP", b200_fhadp.FHADP, b200_fhadp.ApproxContainer)   # INTEGRATION.md section 1
-        alg = ref_ca.create_alg(**dict(kw, use_gpu=True))              # reference factory -> fused algorithm
+        ca.register("FHADP", b200_fhadp.FHADP, b200_fhadp.ApproxContainer)   # INTEGRATION.md section 1
+        alg = ca.create_alg(**dict(kw, use_gpu=True))
     finally:
-        ref_ca.registry["FHADP"] = saved
+        ca.registry["FHADP"] = saved
     assert type(alg).__module__ == "gops_b200.algorithm.fhadp"
-    alg.load_state_dict(ref_alg.state_dict())                          # identical start (reference checkpoint keys)
+    alg.load_state_dict(ref_sd)                                          # identical start (reference checkpoint keys)
 
-    buf = ReplayBuffer(trainer="off_serial_trainer", seed=0, obsv_dim=6, action_dim=1, buffer_max_size=4096,
-                       additional_info={})
-    g = torch.Generator().manual_seed(3)
-    h = torch.tensor([5, 0.1, 0.1, 0.3, 0.3, 0.3])
-    obs = ((torch.rand(2048, 6, generator=g) * 2 - 1) * h).numpy()
-    buf.add_batch([(o, np.zeros(1, np.float32), 0.0, False, {}, o, {}, 0.0) for o in obs])
     for it in range(3):
-        replay = buf.sample_batch(512)
-        ref_tb = ref_alg.local_update({k: v.clone() for k, v in replay.items()}, it)
+        prefix = f"it{it}/batch/"
+        replay = {k[len(prefix):]: torch.from_numpy(v) for k, v in rec.items() if k.startswith(prefix)}
         gpu_batch = {k: v.cuda() for k, v in replay.items()}          # off_serial_trainer.py:92-94
         alg.networks.train()
         tb = alg.local_update(gpu_batch, it)
         alg.networks.eval()
         assert set(tb) >= {"Loss/Actor loss-RL iter", "Time/Algorithm time [ms]-RL iter"}
-        ref_loss = ref_tb["Loss/Actor loss-RL iter"]
+        ref_loss = float(rec[f"it{it}/loss"])
         assert abs(tb["Loss/Actor loss-RL iter"] - ref_loss) <= (1e-4 if it == 0 else 5e-4) * max(1.0, abs(ref_loss))
     # the sampler / evaluator side: the trained policies act alike
-    o = torch.from_numpy(obs[:32])
-    with torch.no_grad():
-        a_ref = ref_alg.networks.policy(o, 1)
+    o = torch.from_numpy(rec["act_obs"])
     a = alg.networks.policy(o.cuda(), 1).cpu()
-    assert float((a - a_ref).abs().max()) < 1e-3
-    # and the checkpoint the fused algorithm writes loads back into the reference
-    ref_alg.load_state_dict({k: v.cpu() for k, v in alg.state_dict().items()})
+    assert float((a - torch.from_numpy(rec["act"])).abs().max()) < 1e-3
+    # and the checkpoint the fused algorithm writes loads back into the reference (a strict load: same keys and shapes)
+    sd = alg.state_dict()
+    assert set(sd) == set(ref_sd)
+    for k, v in ref_sd.items():
+        assert sd[k].shape == v.shape, k
